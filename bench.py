@@ -33,6 +33,8 @@ sys.path.insert(0, ROOT)
 
 BASELINE_GBPS = 0.233  # the only throughput figure in the reference tree (configs/worker.yaml:19, unsourced)
 NVLINK_NOMINAL_GBPS = 900.0  # BASELINE.json: per direction per GPU
+DUMP_SAMPLE_BYTES = 8 << 20  # --dump-outputs: payload bytes sampled over all ranks, 32 MB as float32
+DUMP_SEED = 0xB200
 
 
 def reference_arm() -> int:
@@ -72,7 +74,12 @@ def main() -> int:
                     help="N>1: ranks rendezvous per step / per put-get phase (inside the timed region)")
     ap.add_argument("--idle-odd", action="store_true", help="diagnostic: odd ranks idle (unidirectional NVLink traffic)")
     ap.add_argument("--quick", action="store_true", help="sweep config: fewer sizes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="headline config: after the timed steps, write what the last timed step handed back to its caller as DIR/<name>.npy "
+                         "(a fixed sample of the bytes the get delivered, the get sizes, the put / get status codes)")
     args = ap.parse_args()
+    if args.dump_outputs and args.config != "headline":
+        ap.error("--dump-outputs applies to the headline config")
     if args.impl == "reference":
         return reference_arm()
 
@@ -87,6 +94,7 @@ def main() -> int:
 
 # ====================================================================================================== headline
 def run_headline(args, world: int) -> int:
+    import numpy as np
     import torch
 
     from blackbird_b200 import _bb
@@ -131,15 +139,17 @@ def run_headline(args, world: int) -> int:
         if args.sync != "none":
             rendezvous()  # bulk-synchronous step (checkpoint / KV hand-off pattern): all ranks put, then all ranks get
         if not idle:
-            ecs = cl.client.batch_put_device(keys, put_ptrs or src_ptrs, sizes, c or cfg, stream)
-            assert all(e == OK for e in ecs), f"put failed: {[str(e) for e in ecs if e != OK][:3]}"
+            put_ecs = cl.client.batch_put_device(keys, put_ptrs or src_ptrs, sizes, c or cfg, stream)
+            assert all(e == OK for e in put_ecs), f"put failed: {[str(e) for e in put_ecs if e != OK][:3]}"
         if args.sync == "phase":
             rendezvous()
         if not idle:
-            ecs, _ = cl.client.batch_get_device(keys, get_ptrs or out_ptrs, sizes, stream)
-            assert all(e == OK for e in ecs), f"get failed: {[str(e) for e in ecs if e != OK][:3]}"
+            get_ecs, got = cl.client.batch_get_device(keys, get_ptrs or out_ptrs, sizes, stream)
+            assert all(e == OK for e in get_ecs), f"get failed: {[str(e) for e in get_ecs if e != OK][:3]}"
             ecs = cl.client.batch_remove(keys)
             assert all(e == OK for e in ecs)
+            return put_ecs, get_ecs, got
+        return None
 
     if args.ctas:
         cl.fabric.set_max_ctas(args.ctas)
@@ -159,12 +169,23 @@ def run_headline(args, world: int) -> int:
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        step("t", i, all_keys[i])
+        last = step("t", i, all_keys[i])
     e1.record()
     torch.cuda.synchronize()
     cl.barrier()
     ms = cl.max_over_ranks(e0.elapsed_time(e1))
     launches = int(cl.sum_over_ranks(cl.fabric.launches - launches0))
+    dump = {}
+    if args.dump_outputs and not idle:
+        # Taken now because the phases below reuse `out`; written at the end.  The sample positions depend only on the
+        # batch size, and the sources are seeded, so two builds run with the same arguments dump comparable arrays.
+        put_ecs, get_ecs, got = last
+        n_sample = min(step_bytes, DUMP_SAMPLE_BYTES // world)
+        pick = np.sort(np.random.default_rng(DUMP_SEED).integers(0, step_bytes, n_sample)) if n_sample < step_bytes else np.arange(step_bytes)
+        dump = {"get_bytes_sample": out[torch.from_numpy(pick).to(dev)].float(),
+                "get_sizes": torch.tensor(got, dtype=torch.float64),
+                "put_status": torch.tensor([int(e) for e in put_ecs], dtype=torch.float64),
+                "get_status": torch.tensor([int(e) for e in get_ecs], dtype=torch.float64)}
     if ms < 1500:  # give nvidia-smi time to take samples under the same load (same count on every rank: steps rendezvous)
         for i in range(int(1200.0 / max(ms / args.steps, 0.05)) + 1):
             step("c", i)
@@ -373,6 +394,11 @@ def run_headline(args, world: int) -> int:
             comparators["fused_put_kernel_vs_per_object_cudaMemcpyPeerAsync_without_digest"] = round(
                 kernel_only["put_GBps_per_gpu"] / comparators["per_object_cudaMemcpyPeerAsync_GBps_per_rank"], 3)
 
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        prefix = f"rank{rank}_" if world > 1 else ""
+        for name, t in dump.items():
+            np.save(os.path.join(args.dump_outputs, prefix + name + ".npy"), t.cpu().numpy())
     cl.stop()
     if world > 1 and cl.dist is not None:
         try:

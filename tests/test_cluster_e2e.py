@@ -197,10 +197,11 @@ def test_multi_tier_worker_and_class_preference(bb, tmp_path):
 
 
 def test_config_files_parse(bb, tmp_path):
-    ks = bb.KeystoneConfig.from_yaml("/root/reference/configs/keystone.yaml")  # reference sample parses unchanged
+    reference_configs = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_configs")
+    ks = bb.KeystoneConfig.from_yaml(os.path.join(reference_configs, "keystone.yaml"))  # reference sample parses unchanged
     assert ks.cluster_id == "blackbird_cluster" and ks.etcd_endpoints == "localhost:2379" and ks.high_watermark == 0.8
     assert ks.client_ttl_sec == 300 and ks.max_replicas == 3 and ks.log_level == "INFO"
-    wc = bb.WorkerServiceConfig.from_yaml("/root/reference/configs/worker.yaml")
+    wc = bb.WorkerServiceConfig.from_yaml(os.path.join(reference_configs, "worker.yaml"))
     assert wc.worker_id == "worker-1" and wc.interconnects == ["rdma", "tcp"] and wc.heartbeat_interval_sec == 5
     assert wc.storage_pools[0].pool_id == "ram_pool_0" and wc.storage_pools[0].size_bytes == 2 << 30
     for name in ("keystone.yaml", "worker.yaml", "gpu_worker.yaml", "tiered_worker.yaml"):

@@ -4,6 +4,8 @@ import os
 import numpy as np
 import pytest
 
+REFERENCE_CONFIGS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_configs")
+
 
 def test_error_codes_domains_and_strings(bb):
     E = bb.ErrorCode
@@ -31,15 +33,15 @@ def test_json_roundtrip_and_errors(bb):
 
 
 def test_yaml_reference_configs(bb):
-    ks = bb.parse_yaml(open("/root/reference/configs/keystone.yaml").read())
+    ks = bb.parse_yaml(open(os.path.join(REFERENCE_CONFIGS, "keystone.yaml")).read())
     assert ks["keystone"]["cluster_id"] == "blackbird_cluster"
     assert ks["keystone"]["etcd_endpoints"] == ["localhost:2379"]
     assert ks["keystone"]["high_watermark"] == 0.8 and ks["keystone"]["enable_ha"] is False
     assert ks["logging"]["level"] == "INFO"
-    w = bb.parse_yaml(open("/root/reference/configs/worker.yaml").read())
+    w = bb.parse_yaml(open(os.path.join(REFERENCE_CONFIGS, "worker.yaml")).read())
     assert w["worker"]["interconnects"] == ["rdma", "tcp"]
     assert w["storage_pools"][0] == {"pool_id": "ram_pool_0", "storage_class": "RAM_CPU", "size_bytes": 2147483648}
-    cxl = bb.parse_yaml(open("/root/reference/configs/cxl_worker.yaml").read())
+    cxl = bb.parse_yaml(open(os.path.join(REFERENCE_CONFIGS, "cxl_worker.yaml")).read())
     pools = cxl["worker"]["storage_pools"]
     assert pools[1]["config"]["dax_device"] == "/dev/dax0.0" and pools[1]["capacity"] == "256_GB"
     assert cxl["worker"]["allocation"]["preferred_tiers"][3]["max_size"] == "unlimited"

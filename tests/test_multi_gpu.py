@@ -39,7 +39,7 @@ def test_ring_replication_fanout_and_remote_dram_on_n_gpus():
 
     n = torch.cuda.device_count()
     if n < 2:
-        pytest.skip("needs >= 2 GPUs (run under `gpurun --gpus 2`)")
+        pytest.skip("needs >= 2 GPUs")
     world = min(n, 4)
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}", "--master-addr", "127.0.0.1",
            "--master-port", str(_free_port()), os.path.join(ROOT, "tests", "multi_gpu_worker.py")]
