@@ -8,6 +8,7 @@
 
 #include <cstdint>
 
+#include "kernels/mxfp8.cuh"
 #include "kernels/ptx.cuh"
 #include "kernels/xfer.h"
 
@@ -64,7 +65,7 @@ __global__ void __launch_bounds__(256) mxfp8_unpack_kernel(const uint2* __restri
   const uint64_t n = nblocks * 4;
   for (uint64_t t = static_cast<uint64_t>(blockIdx.x) * blockDim.x + threadIdx.x; t < n; t += stride) {
     const uint2 p = payload[t];
-    const float s = __int_as_float(static_cast<int>(scales[t >> 2]) << 23);  // 2^(e-127); e==0 -> 0 (flush)
+    const float s = e8m0_scale(scales[t >> 2]);
     uint32_t out[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {

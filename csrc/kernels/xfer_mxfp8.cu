@@ -26,6 +26,7 @@
 #include <mutex>
 
 #include "common/tchash_def.h"
+#include "kernels/mxfp8.cuh"
 #include "kernels/ptx.cuh"
 #include "kernels/xfer.h"
 
@@ -147,7 +148,7 @@ __device__ __forceinline__ void pack_chunk(const uint4 v, uint2* payload_out, ui
 }
 
 __device__ __forceinline__ uint4 unpack_chunk(const uint2 p, uint8_t scale) {
-  const float s = __int_as_float(static_cast<int>(scale) << 23);  // 2^(e-127); e == 0 flushes to zero
+  const float s = e8m0_scale(scale);
   auto cvt2 = [&](uint32_t two) -> uint32_t {  // two E4M3 bytes -> bf16x2
     const __half2_raw hr = __nv_cvt_fp8x2_to_halfraw2(static_cast<__nv_fp8x2_storage_t>(two & 0xFFFFu), __NV_E4M3);
     const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&hr));

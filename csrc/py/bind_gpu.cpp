@@ -80,9 +80,19 @@ void bind_gpu(py::module_& m) {
              std::vector<gpu::Fp8Item> v;
              for (auto h : items) {
                auto t = h.cast<py::tuple>();
+               if (t.size() < 3) throw py::value_error("fp8 item = (bf16, packed|[packed..], n_elems[, expect])");
                gpu::Fp8Item it;
                it.wide = reinterpret_cast<void*>(t[0].cast<uintptr_t>());
-               it.packed = reinterpret_cast<void*>(t[1].cast<uintptr_t>());
+               if (py::isinstance<py::int_>(t[1])) {
+                 it.packed = reinterpret_cast<void*>(t[1].cast<uintptr_t>());
+               } else {
+                 auto p = t[1].cast<std::vector<uintptr_t>>();
+                 if (p.empty() || p.size() > kMaxDst) throw py::value_error("1..3 packed replicas");
+                 if (unpack && p.size() > 1) throw py::value_error("a get reads one packed copy");
+                 it.packed = reinterpret_cast<void*>(p[0]);
+                 for (size_t r = 1; r < p.size(); ++r) it.more_packed[r - 1] = reinterpret_cast<void*>(p[r]);
+                 it.nreplicas = static_cast<uint32_t>(p.size());
+               }
                it.n_elems = t[2].cast<uint64_t>();
                if (t.size() > 3) it.expect = t[3].cast<uint64_t>(), it.verify = true;
                v.push_back(it);
@@ -95,8 +105,9 @@ void bind_gpu(py::module_& m) {
              return py::make_tuple(res.digest, res.status, res.device_ms);
            },
            py::arg("items"), py::arg("unpack"), py::arg("stream") = 0,
-           "Fused MXFP8 put (unpack=False: bf16 -> packed slab object) or get (unpack=True); items = (bf16_ptr, packed_ptr, "
-           "n_elems[, expected_digest]); returns (digests of the packed objects, status, device_ms).")
+           "Fused MXFP8 put (unpack=False: bf16 -> packed slab object) or get (unpack=True); items = (bf16_ptr, packed_ptr | "
+           "[packed_ptr, ...], n_elems[, expected_digest]); a put writes every listed replica (1..3), a get reads one; "
+           "returns (digests of the packed objects, status, device_ms).")
       .def_static("fp8_eligible", &XferEngine::fp8_eligible)
       .def("submit",
            [](XferEngine& e, const py::list& items, ChecksumAlgo algo, uintptr_t stream) {
