@@ -156,6 +156,81 @@ class TensorStore:
     def get(self, key: str, device: Optional[torch.device] = None) -> torch.Tensor:
         return self.batch_get([key], device)[0]
 
+    # ------------------------------------------------------------------ paged KV blocks
+    @staticmethod
+    def _block_segments(caches: Sequence[torch.Tensor], block_ids: Sequence[torch.Tensor]):
+        """(S, 2) int64 segment table (pointer, bytes) and per-object segment counts: object i is, cache by cache in list
+        order, caches[c][block_ids[i][j]] for every j."""
+        if not caches:
+            raise ValueError("batch_*_blocks needs at least one cache tensor")
+        bases, strides, lens, nblocks = [], [], [], []
+        for c in caches:
+            if not c.is_cuda:
+                raise ValueError("caches must be CUDA tensors")
+            if c.dim() < 1 or c.shape[0] == 0:
+                raise ValueError(f"a cache is [num_blocks, ...]; got shape {tuple(c.shape)}")
+            if not c[0].is_contiguous():
+                raise ValueError(f"each cache must be contiguous in its trailing dimensions (shape {tuple(c.shape)}, stride {c.stride()})")
+            es = c.element_size()
+            block = c[0].numel() * es
+            if c.data_ptr() % 16 or (c.stride(0) * es) % 16 or block % 16:
+                raise ValueError(f"cache blocks must start 16-byte aligned and be a multiple of 16 bytes (block {block} B, "
+                                 f"stride {c.stride(0) * es} B, base {c.data_ptr():#x})")
+            bases.append(c.data_ptr())
+            strides.append(c.stride(0) * es)
+            lens.append(block)
+            nblocks.append(c.shape[0])
+        bases = torch.tensor(bases, dtype=torch.int64)[:, None]
+        strides = torch.tensor(strides, dtype=torch.int64)[:, None]
+        lens = torch.tensor(lens, dtype=torch.int64)[:, None]
+        limit = min(nblocks)
+        rows, counts = [], []
+        for ids in block_ids:
+            ids = torch.as_tensor(ids).to("cpu", torch.int64).reshape(-1)
+            if ids.numel() == 0:
+                raise ValueError("every key needs at least one block")
+            if int(ids.min()) < 0 or int(ids.max()) >= limit:
+                raise IndexError(f"block index out of range [0, {limit})")
+            ptr = bases + ids[None, :] * strides                      # [cache, block]
+            rows.append(torch.stack([ptr.reshape(-1), lens.expand(-1, ids.numel()).reshape(-1)], 1))
+            counts.append(ptr.numel())
+        return torch.cat(rows), counts
+
+    def batch_put_blocks(self, keys: Sequence[str], caches: Sequence[torch.Tensor], block_ids: Sequence[torch.Tensor], config=None) -> None:
+        """Stores object keys[i] = the blocks block_ids[i] of every cache (cache by cache, in list order) with one fused
+        gather put: no staging copy.  The object is the same as a contiguous put of those blocks concatenated, so
+        `get` returns it as a flat uint8 tensor and `remove` / `keys` work on it."""
+        keys = list(keys)
+        if len(keys) != len(block_ids):
+            raise ValueError("one block list per key")
+        cfg = config or self.config
+        segs, counts = self._block_segments(caches, block_ids)
+        ecs = self.client.batch_put_device_gather(keys, segs, counts, cfg, self._stream())
+        bad = [(k, e) for k, e in zip(keys, ecs) if e != _bb.ErrorCode.OK]
+        if bad:
+            raise RuntimeError(f"block put failed: {bad[:3]}")
+        sizes, pos = [], 0
+        for n in counts:
+            sizes.append(int(segs[pos:pos + n, 1].sum()))
+            pos += n
+        metas = [json.dumps({"dtype": "uint8", "shape": [s], "packed": None, "numel": s}).encode() for s in sizes]
+        ecs = self.client.batch_put([k + "#meta" for k in keys], metas, self._meta_cfg())
+        if any(e != _bb.ErrorCode.OK for e in ecs):
+            raise RuntimeError("meta put failed")
+
+    def batch_get_blocks(self, keys: Sequence[str], caches: Sequence[torch.Tensor], block_ids: Sequence[torch.Tensor]) -> None:
+        """Writes object keys[i] into the blocks block_ids[i] of every cache (the layout of batch_put_blocks; the block
+        ids may differ from the ones it was stored from) with one fused scatter get.  The blocks must add up to the
+        stored size.  Block lists that overlap receive unspecified bytes."""
+        keys = list(keys)
+        if len(keys) != len(block_ids):
+            raise ValueError("one block list per key")
+        segs, counts = self._block_segments(caches, block_ids)
+        ecs = self.client.batch_get_device_scatter(keys, segs, counts, self._stream())
+        bad = [(k, e) for k, e in zip(keys, ecs) if e != _bb.ErrorCode.OK]
+        if bad:
+            raise RuntimeError(f"block get failed: {bad[:3]}")
+
     def remove(self, keys: Sequence[str]) -> None:
         self.client.batch_remove(list(keys) + [k + "#meta" for k in keys])
 
@@ -209,6 +284,36 @@ class AsyncTensorStore(TensorStore):
                 out = self.batch_get(keys)
             self._side.synchronize()
             return out
+
+        return self._pool.submit(run)
+
+    def put_blocks_async(self, keys: Sequence[str], caches: Sequence[torch.Tensor], block_ids: Sequence[torch.Tensor], config=None):
+        ready = torch.cuda.Event()
+        ready.record(torch.cuda.current_stream())  # the blocks' producers
+        caches, block_ids = list(caches), list(block_ids)
+
+        def run():
+            torch.cuda.set_device(self._device)
+            self._side.wait_event(ready)
+            with torch.cuda.stream(self._side):
+                self.batch_put_blocks(keys, caches, block_ids, config)
+            self._side.synchronize()
+            return len(keys)
+
+        return self._pool.submit(run)
+
+    def get_blocks_async(self, keys: Sequence[str], caches: Sequence[torch.Tensor], block_ids: Sequence[torch.Tensor]):
+        ready = torch.cuda.Event()
+        ready.record(torch.cuda.current_stream())  # work queued on the destination blocks so far
+        caches, block_ids = list(caches), list(block_ids)
+
+        def run():
+            torch.cuda.set_device(self._device)
+            self._side.wait_event(ready)
+            with torch.cuda.stream(self._side):
+                self.batch_get_blocks(keys, caches, block_ids)
+            self._side.synchronize()
+            return len(keys)
 
         return self._pool.submit(run)
 

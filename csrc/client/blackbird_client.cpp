@@ -891,8 +891,88 @@ static void ewma_update(std::atomic<double>& v, double sample) {
   v.store(old == 0 ? sample : 0.75 * old + 0.25 * sample, std::memory_order_relaxed);
 }
 
+// Segment table entries one chunk of a segmented batch may hand to the transport (one fused launch each).
+static constexpr size_t kMaxChunkSegments = size_t{1} << 20;
+
+// Splits chunks further so that none carries more than kMaxChunkSegments segments (a chunk keeps at least one object).
+static std::vector<std::pair<size_t, size_t>> cap_chunk_segments(const std::vector<std::pair<size_t, size_t>>& plan,
+                                                                 const std::vector<size_t>& count) {
+  std::vector<std::pair<size_t, size_t>> out;
+  for (const auto& [b, e] : plan) {
+    size_t begin = b, acc = 0;
+    for (size_t i = b; i < e; ++i) {
+      if (i > begin && acc + count[i] > kMaxChunkSegments) {
+        out.emplace_back(begin, i);
+        begin = i, acc = 0;
+      }
+      acc += count[i];
+    }
+    out.emplace_back(begin, e);
+  }
+  return out;
+}
+
+// Checks the segment rules object by object.  verdict[i] = OK for a valid object (its total length in total[i]); false
+// when seg_counts do not add up to segs.size() (the whole batch is invalid).
+static bool index_segments(const std::vector<DeviceSegment>& segs, const std::vector<uint32_t>& seg_counts, std::vector<size_t>* first,
+                           std::vector<ErrorCode>* verdict, std::vector<size_t>* total) {
+  uint64_t sum = 0;
+  for (uint32_t c : seg_counts) sum += c;
+  if (sum != segs.size()) return false;
+  first->assign(seg_counts.size(), 0);
+  total->assign(seg_counts.size(), 0);
+  size_t pos = 0;
+  for (size_t i = 0; i < seg_counts.size(); ++i) {
+    const size_t n = seg_counts[i];
+    (*first)[i] = pos;
+    bool ok = n > 0;
+    uint64_t bytes = 0;
+    for (size_t k = 0; k < n && ok; ++k) {
+      const DeviceSegment& s = segs[pos + k];
+      ok = (s.ptr & 15) == 0 && s.len > 0 && (k + 1 == n || (s.len & 15) == 0);
+      bytes += s.len;
+    }
+    pos += n;
+    (*verdict)[i] = !ok ? ErrorCode::INVALID_PARAMETERS
+                    : n > BlackbirdClient::kMaxObjectSegments ? ErrorCode::VALUE_OUT_OF_RANGE : ErrorCode::OK;
+    (*total)[i] = bytes;
+  }
+  return true;
+}
+
 std::vector<ErrorCode> BlackbirdClient::batch_put_device(const std::vector<ObjectKey>& keys, const std::vector<const void*>& dev_ptrs,
                                                          const std::vector<size_t>& sizes, const WorkerConfig& cfg, void* stream) {
+  return put_device_impl(keys, dev_ptrs, sizes, nullptr, cfg, stream);
+}
+
+std::vector<ErrorCode> BlackbirdClient::batch_put_device_gather(const std::vector<ObjectKey>& keys, const std::vector<DeviceSegment>& segs,
+                                                                const std::vector<uint32_t>& seg_counts, const WorkerConfig& cfg,
+                                                                void* stream) {
+  std::vector<ErrorCode> out(keys.size(), ErrorCode::INVALID_PARAMETERS);
+  if (!keystone_) return std::vector<ErrorCode>(keys.size(), ErrorCode::CLIENT_DISCONNECTED);
+  if (!device_) return std::vector<ErrorCode>(keys.size(), ErrorCode::NOT_IMPLEMENTED);
+  std::vector<size_t> first, total;
+  if (seg_counts.size() != keys.size() || !index_segments(segs, seg_counts, &first, &out, &total))
+    return std::vector<ErrorCode>(keys.size(), ErrorCode::INVALID_PARAMETERS);
+  // the valid objects go on as one batch; the others keep their verdict
+  SegView sv;
+  sv.segs = segs.data();
+  std::vector<ObjectKey> vkeys;
+  std::vector<size_t> idx, sizes;
+  for (size_t i = 0; i < keys.size(); ++i) {
+    if (out[i] != ErrorCode::OK) continue;
+    idx.push_back(i), vkeys.push_back(keys[i]), sizes.push_back(total[i]);
+    sv.first.push_back(first[i]), sv.count.push_back(seg_counts[i]);
+  }
+  if (idx.empty()) return out;
+  auto r = put_device_impl(vkeys, std::vector<const void*>(idx.size(), nullptr), sizes, &sv, cfg, stream);
+  for (size_t k = 0; k < idx.size(); ++k) out[idx[k]] = r[k];
+  return out;
+}
+
+std::vector<ErrorCode> BlackbirdClient::put_device_impl(const std::vector<ObjectKey>& keys, const std::vector<const void*>& dev_ptrs,
+                                                        const std::vector<size_t>& sizes, const SegView* sv, const WorkerConfig& cfg,
+                                                        void* stream) {
   std::vector<ErrorCode> out(keys.size(), ErrorCode::INVALID_PARAMETERS);
   if (!keystone_) return std::vector<ErrorCode>(keys.size(), ErrorCode::CLIENT_DISCONNECTED);
   if (!device_) return std::vector<ErrorCode>(keys.size(), ErrorCode::NOT_IMPLEMENTED);
@@ -908,7 +988,8 @@ std::vector<ErrorCode> BlackbirdClient::batch_put_device(const std::vector<Objec
     bool submitted = false;
     ErrorCode submit_error = ErrorCode::OK;
   };
-  const auto plan = plan_chunks(sizes, put_rpc_us_per_obj_.load(std::memory_order_relaxed));
+  auto plan = plan_chunks(sizes, put_rpc_us_per_obj_.load(std::memory_order_relaxed));
+  if (sv) plan = cap_chunk_segments(plan, sv->count);
   double rpc_us_total = 0;
   std::vector<Chunk> chunks(plan.size());
   std::vector<size_t> host_put;                      // objects whose placement is not on the GPU fabric
@@ -963,6 +1044,7 @@ std::vector<ErrorCode> BlackbirdClient::batch_put_device(const std::vector<Objec
           op.shard = s;
           op.placement = &copies[0].shards[s];
           op.obj_offset = off;
+          if (sv) op.segs = sv->segs + sv->first[i], op.nsegs = sv->count[i];
           for (size_t c = 1; c < copies.size(); ++c) op.replicas.push_back(&copies[c].shards[s]);
           ch.ops.push_back(std::move(op));
           off += copies[0].shards[s].length;
@@ -977,6 +1059,7 @@ std::vector<ErrorCode> BlackbirdClient::batch_put_device(const std::vector<Objec
             op.shard = s;
             op.placement = &copies[c].shards[s];
             op.obj_offset = o2;
+            if (sv) op.segs = sv->segs + sv->first[i], op.nsegs = sv->count[i];
             ch.ops.push_back(std::move(op));
             o2 += copies[c].shards[s].length;
           }
@@ -1054,7 +1137,17 @@ std::vector<ErrorCode> BlackbirdClient::batch_put_device(const std::vector<Objec
   // host-tier placements: D2H into a staging buffer, then the TCP data path (checksums on the CPU)
   for (size_t i : host_put) {
     std::vector<uint8_t> stage(sizes[i]);
-    ErrorCode ec = device_->copy_d2h(stage.data(), dev_ptrs[i], sizes[i], stream);
+    ErrorCode ec = ErrorCode::OK;
+    if (sv) {  // gather: one D2H per segment
+      uint64_t pos = 0;
+      for (size_t k = 0; k < sv->count[i] && ec == ErrorCode::OK; ++k) {
+        const DeviceSegment& sg = sv->segs[sv->first[i] + k];
+        ec = device_->copy_d2h(stage.data() + pos, reinterpret_cast<const void*>(sg.ptr), sg.len, stream);
+        pos += sg.len;
+      }
+    } else {
+      ec = device_->copy_d2h(stage.data(), dev_ptrs[i], sizes[i], stream);
+    }
     ShardChecksums sums;
     if (ec == ErrorCode::OK) ec = transfer_put(host_placed[i], stage.data(), cfg.checksum, &sums);
     if (ec == ErrorCode::OK) ec = keystone_->put_complete(keys[i], sums);
@@ -1071,6 +1164,35 @@ std::vector<ErrorCode> BlackbirdClient::batch_put_device(const std::vector<Objec
 std::vector<ErrorCode> BlackbirdClient::batch_get_device(const std::vector<ObjectKey>& keys, const std::vector<void*>& dev_ptrs,
                                                          const std::vector<size_t>& capacity, void* stream,
                                                          std::vector<size_t>* out_sizes) {
+  return get_device_impl(keys, dev_ptrs, capacity, nullptr, stream, out_sizes);
+}
+
+std::vector<ErrorCode> BlackbirdClient::batch_get_device_scatter(const std::vector<ObjectKey>& keys, const std::vector<DeviceSegment>& segs,
+                                                                 const std::vector<uint32_t>& seg_counts, void* stream) {
+  std::vector<ErrorCode> out(keys.size(), ErrorCode::INVALID_PARAMETERS);
+  if (!keystone_) return std::vector<ErrorCode>(keys.size(), ErrorCode::CLIENT_DISCONNECTED);
+  if (!device_) return std::vector<ErrorCode>(keys.size(), ErrorCode::NOT_IMPLEMENTED);
+  std::vector<size_t> first, total;
+  if (seg_counts.size() != keys.size() || !index_segments(segs, seg_counts, &first, &out, &total))
+    return std::vector<ErrorCode>(keys.size(), ErrorCode::INVALID_PARAMETERS);
+  SegView sv;
+  sv.segs = segs.data();
+  std::vector<ObjectKey> vkeys;
+  std::vector<size_t> idx, caps;
+  for (size_t i = 0; i < keys.size(); ++i) {
+    if (out[i] != ErrorCode::OK) continue;
+    idx.push_back(i), vkeys.push_back(keys[i]), caps.push_back(total[i]);
+    sv.first.push_back(first[i]), sv.count.push_back(seg_counts[i]);
+  }
+  if (idx.empty()) return out;
+  auto r = get_device_impl(vkeys, std::vector<void*>(idx.size(), nullptr), caps, &sv, stream, nullptr);
+  for (size_t k = 0; k < idx.size(); ++k) out[idx[k]] = r[k];
+  return out;
+}
+
+std::vector<ErrorCode> BlackbirdClient::get_device_impl(const std::vector<ObjectKey>& keys, const std::vector<void*>& dev_ptrs,
+                                                        const std::vector<size_t>& capacity, const SegView* sv, void* stream,
+                                                        std::vector<size_t>* out_sizes) {
   std::vector<ErrorCode> out(keys.size(), ErrorCode::INVALID_PARAMETERS);
   if (!keystone_) return std::vector<ErrorCode>(keys.size(), ErrorCode::CLIENT_DISCONNECTED);
   if (!device_) return std::vector<ErrorCode>(keys.size(), ErrorCode::NOT_IMPLEMENTED);
@@ -1095,6 +1217,7 @@ std::vector<ErrorCode> BlackbirdClient::batch_get_device(const std::vector<Objec
         op.shard = s;
         op.placement = &copy.shards[s];
         op.obj_offset = off;
+        if (sv) op.segs = sv->segs + sv->first[i], op.nsegs = sv->count[i];
         ops.push_back(std::move(op));
         off += copy.shards[s].length;
       }
@@ -1127,7 +1250,8 @@ std::vector<ErrorCode> BlackbirdClient::batch_get_device(const std::vector<Objec
     bool submitted = false;
     ErrorCode err = ErrorCode::OK;
   };
-  const auto plan = plan_chunks(capacity, get_rpc_us_per_obj_.load(std::memory_order_relaxed));
+  auto plan = plan_chunks(capacity, get_rpc_us_per_obj_.load(std::memory_order_relaxed));
+  if (sv) plan = cap_chunk_segments(plan, sv->count);
   double rpc_us_total = 0;
   std::vector<Chunk> chunks(plan.size());
   std::vector<size_t> retry;
@@ -1176,6 +1300,10 @@ std::vector<ErrorCode> BlackbirdClient::batch_get_device(const std::vector<Objec
       size_t size = 0;
       for (const auto& s : placed[i].value()[0].shards) size += s.length;
       if (out_sizes) (*out_sizes)[i] = size;
+      if (sv && size != capacity[i]) {  // a scatter list must cover the object exactly
+        out[i] = ErrorCode::INVALID_PARAMETERS;
+        continue;
+      }
       if (size > capacity[i]) {
         out[i] = ErrorCode::BUFFER_OVERFLOW;
         continue;
@@ -1211,7 +1339,16 @@ std::vector<ErrorCode> BlackbirdClient::batch_get_device(const std::vector<Objec
       if (!found) {
         std::vector<uint8_t> stage(size);
         ErrorCode ec = transfer_get(copies, stage.data(), size);  // data servers + CPU checksum + replica fail-over
-        if (ec == ErrorCode::OK) ec = device_->copy_h2d(dev_ptrs[i], stage.data(), size, stream);
+        if (ec == ErrorCode::OK && sv) {  // scatter: one H2D per segment
+          uint64_t pos = 0;
+          for (size_t k = 0; k < sv->count[i] && ec == ErrorCode::OK; ++k) {
+            const DeviceSegment& sg = sv->segs[sv->first[i] + k];
+            ec = device_->copy_h2d(reinterpret_cast<void*>(sg.ptr), stage.data() + pos, sg.len, stream);
+            pos += sg.len;
+          }
+        } else if (ec == ErrorCode::OK) {
+          ec = device_->copy_h2d(dev_ptrs[i], stage.data(), size, stream);
+        }
         out[i] = ec;
         metrics_.inc("device_get_host_staged_total");
         continue;
@@ -1302,6 +1439,8 @@ std::vector<ErrorCode> BlackbirdClient::batch_get_device(const std::vector<Objec
       std::vector<ObjectKey> rkeys;
       std::vector<void*> rptrs;
       std::vector<size_t> rcaps, ridx;
+      SegView rsv;
+      if (sv) rsv.segs = sv->segs;
       for (size_t k = 0; k < bad.size(); ++k) {
         const size_t i = bad[k];
         if (!again[k].ok()) {
@@ -1310,13 +1449,14 @@ std::vector<ErrorCode> BlackbirdClient::batch_get_device(const std::vector<Objec
           // changed placements, or (once) the same ones: a remove + re-put can land on the very same extent (first fit)
           // and be read half-written
           rkeys.push_back(keys[i]), rptrs.push_back(dev_ptrs[i]), rcaps.push_back(capacity[i]), ridx.push_back(i);
+          if (sv) rsv.first.push_back(sv->first[i]), rsv.count.push_back(sv->count[i]);
         }
       }
       if (!rkeys.empty()) {
         metrics_.inc("get_placement_refresh_total", rkeys.size());
         std::vector<size_t> rsizes;
         ++refresh_depth;
-        auto recs = batch_get_device(rkeys, rptrs, rcaps, stream, &rsizes);
+        auto recs = get_device_impl(rkeys, rptrs, rcaps, sv ? &rsv : nullptr, stream, &rsizes);
         --refresh_depth;
         for (size_t k = 0; k < ridx.size(); ++k) {
           out[ridx[k]] = recs[k];
@@ -1341,9 +1481,15 @@ ErrorCode HostLoopbackTransport::put_shards(const std::vector<DeviceShardOp>& op
                                             void*, std::vector<uint64_t>* digests) {
   ++launches_;  // one "launch" per batch, like the fused kernel
   if (digests) digests->assign(ops.size(), 0);
+  std::vector<uint8_t> gathered;
   for (size_t k = 0; k < ops.size(); ++k) {
     const DeviceShardOp& op = ops[k];
     const auto* src = static_cast<const uint8_t*>(dev_ptrs[op.item]) + op.obj_offset;
+    if (op.segs) {  // gather this shard's slice of the segment list
+      gathered.resize(op.placement->length);
+      BB_TRY(copy_segments(op, gathered.data(), true));
+      src = gathered.data();
+    }
     uint64_t d = 0;
     ErrorCode ec = io_->write_shard(*op.placement, src, &d, algo);
     for (size_t r = 0; r < op.replicas.size() && ec == ErrorCode::OK; ++r) ec = io_->write_shard(*op.replicas[r], src, nullptr, ChecksumAlgo::NONE);
@@ -1357,17 +1503,40 @@ ErrorCode HostLoopbackTransport::get_shards(const std::vector<DeviceShardOp>& op
                                             std::vector<uint32_t>* status) {
   ++launches_;
   if (status) status->assign(ops.size(), 0);
+  std::vector<uint8_t> stage;
   for (size_t k = 0; k < ops.size(); ++k) {
     const DeviceShardOp& op = ops[k];
     auto* dst = static_cast<uint8_t*>(dev_ptrs[op.item]) + op.obj_offset;
+    if (op.segs) {
+      stage.resize(op.placement->length);
+      dst = stage.data();
+    }
     const ErrorCode ec = io_->read_shard(*op.placement, dst, op.placement->checksum_algo);
     if (ec == ErrorCode::CHECKSUM_MISMATCH) {
       if (status) (*status)[k] = 1;  // reported per shard, like the kernel's verify flag
+      if (op.segs) BB_TRY(copy_segments(op, stage.data(), false));  // the kernel stores what it read, verified or not
     } else if (ec != ErrorCode::OK) {
       return ec;
+    } else if (op.segs) {
+      BB_TRY(copy_segments(op, stage.data(), false));  // scatter
     }
   }
   return ErrorCode::OK;
+}
+
+ErrorCode HostLoopbackTransport::copy_segments(const DeviceShardOp& op, uint8_t* buf, bool gather) {
+  size_t k = 0;
+  uint64_t skip = 0, left = op.placement->length;
+  if (left == 0) return ErrorCode::OK;
+  if (!segment_slice(op.segs, op.nsegs, op.obj_offset, &k, &skip)) return ErrorCode::INVALID_ARGUMENT;
+  for (; k < op.nsegs && left; ++k, skip = 0) {
+    const uint64_t n = std::min<uint64_t>(op.segs[k].len - skip, left);
+    auto* seg = reinterpret_cast<uint8_t*>(op.segs[k].ptr) + skip;
+    if (gather) std::memcpy(buf, seg, n);
+    else std::memcpy(seg, buf, n);
+    buf += n, left -= n;
+  }
+  return left ? ErrorCode::INVALID_ARGUMENT : ErrorCode::OK;
 }
 
 ErrorCode HostLoopbackTransport::put_fp8(const std::vector<DeviceFp8Op>& ops, void*, std::vector<uint64_t>* digests) {

@@ -55,7 +55,24 @@ struct DeviceShardOp {
   const ShardPlacement* placement = nullptr;
   std::vector<const ShardPlacement*> replicas;  // same shard on the other copies (put fan-out)
   uint64_t obj_offset = 0;    // byte offset of this shard inside the object
+  // Segmented object (gather put / scatter get): the object's whole segment list, or null for a contiguous object at
+  // dev_ptrs[item].  The transport moves the slice [obj_offset, obj_offset + placement->length) of it.
+  const DeviceSegment* segs = nullptr;
+  size_t nsegs = 0;
 };
+
+// Finds the slice [offset, offset + length) of a segment list: index of its first segment and the bytes of that segment
+// before the slice (the slice runs on through the following segments).  Returns false when the list is too short.
+inline bool segment_slice(const DeviceSegment* segs, size_t nsegs, uint64_t offset, size_t* first, uint64_t* skip) {
+  uint64_t pos = 0;
+  for (size_t k = 0; k < nsegs; pos += segs[k].len, ++k)
+    if (offset < pos + segs[k].len) {
+      *first = k;
+      *skip = offset - pos;
+      return true;
+    }
+  return false;
+}
 
 // One object of a fused MXFP8 transfer: the whole packed object ([E4M3 payload][E8M0 scales]) is a single shard.
 struct DeviceFp8Op {
@@ -176,6 +193,19 @@ class BlackbirdClient {
   // out_sizes[i] receives the object size; buffers must be large enough (capacity[i]).
   std::vector<ErrorCode> batch_get_device(const std::vector<ObjectKey>& keys, const std::vector<void*>& dev_ptrs,
                                           const std::vector<size_t>& capacity, void* stream, std::vector<size_t>* out_sizes);
+  // Segmented objects (a paged KV cache: one object = many blocks spread over many tensors).  Object i is the
+  // concatenation of the next seg_counts[i] entries of `segs`; it is stored exactly as a contiguous put of that
+  // concatenation would store it (same bytes, same digests), so every other read / write path works on it.
+  // Each segment: ptr 16-byte aligned, len > 0, len % 16 == 0 except for the object's last segment; at most
+  // kMaxObjectSegments segments per object.  An object breaking these rules is INVALID_PARAMETERS (VALUE_OUT_OF_RANGE
+  // for too many segments) and the rest of the batch proceeds; seg_counts that do not add up to segs.size() make the
+  // whole batch INVALID_PARAMETERS.  Get: the stored size must equal the sum of the segment lengths (else
+  // INVALID_PARAMETERS, nothing written).  Overlapping scatter destinations receive unspecified bytes.
+  static constexpr size_t kMaxObjectSegments = size_t{1} << 20;
+  std::vector<ErrorCode> batch_put_device_gather(const std::vector<ObjectKey>& keys, const std::vector<DeviceSegment>& segs,
+                                                 const std::vector<uint32_t>& seg_counts, const WorkerConfig& cfg, void* stream);
+  std::vector<ErrorCode> batch_get_device_scatter(const std::vector<ObjectKey>& keys, const std::vector<DeviceSegment>& segs,
+                                                  const std::vector<uint32_t>& seg_counts, void* stream);
 
   Result<ClusterStats> cluster_stats();
   rpc::KeystoneApi& keystone() { return *keystone_; }
@@ -201,6 +231,17 @@ class BlackbirdClient {
   // [begin, end) index ranges that split a batch so that transfers of one chunk overlap the
   // control-plane round trips of its neighbours (large batches only).
   std::vector<std::pair<size_t, size_t>> plan_chunks(const std::vector<size_t>& sizes, double rpc_us_per_object) const;
+  // Segment lists of a segmented batch: object i is segs[first[i] .. first[i] + count[i]).
+  struct SegView {
+    const DeviceSegment* segs = nullptr;
+    std::vector<size_t> first, count;
+  };
+  // Bodies of batch_{put,get}_device and of their segmented variants (`sv` null = contiguous objects at dev_ptrs).
+  std::vector<ErrorCode> put_device_impl(const std::vector<ObjectKey>& keys, const std::vector<const void*>& dev_ptrs,
+                                         const std::vector<size_t>& sizes, const SegView* sv, const WorkerConfig& cfg, void* stream);
+  std::vector<ErrorCode> get_device_impl(const std::vector<ObjectKey>& keys, const std::vector<void*>& dev_ptrs,
+                                         const std::vector<size_t>& capacity, const SegView* sv, void* stream,
+                                         std::vector<size_t>* out_sizes);
 
   // Mapped shared DRAM pools (same-host fast path); a mapping is dropped when the pool re-registers under a new key.
   struct ShmPool {
@@ -256,6 +297,8 @@ class HostLoopbackTransport : public DeviceTransport {
   ErrorCode get_fp8(const std::vector<DeviceFp8Op>& ops, void* stream, std::vector<uint32_t>* status) override;
 
  private:
+  // Segmented op: copies the shard's slice of the segment list into (gather) or out of (scatter) `buf`.
+  static ErrorCode copy_segments(const DeviceShardOp& op, uint8_t* buf, bool gather);
   std::shared_ptr<BlackbirdClient> io_;
   bool reach_disk_;
   std::atomic<uint64_t> launches_{0};

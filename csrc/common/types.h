@@ -26,6 +26,13 @@
 namespace bb {
 
 using ObjectKey = std::string;
+
+// `len` bytes at device (or device-accessible) address `ptr`: one piece of a segmented object, whose bytes are the
+// concatenation of its segments (BlackbirdClient::batch_put_device_gather / batch_get_device_scatter).
+struct DeviceSegment {
+  uint64_t ptr = 0;
+  uint64_t len = 0;
+};
 using Version = uint64_t;
 using MemoryPoolId = std::string;
 using NodeId = std::string;

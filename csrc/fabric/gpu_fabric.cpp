@@ -529,14 +529,34 @@ ErrorCode GpuFabric::copy_d2h(void* host, const void* dev, size_t n, void* strea
   return ErrorCode::OK;
 }
 
+// Segmented object: the item moves the slice of the object's segment list that this shard covers (the first and last
+// segment trimmed by the engine), as the gather source (put) or the scatter destination (get).
+static ErrorCode attach_segments(const client::DeviceShardOp& op, uint32_t flag, XferItem* it) {
+  size_t first = 0, last = 0;
+  uint64_t skip = 0, unused = 0;
+  if (it->nbytes == 0) return ErrorCode::OK;
+  if (!client::segment_slice(op.segs, op.nsegs, op.obj_offset, &first, &skip) ||
+      !client::segment_slice(op.segs, op.nsegs, op.obj_offset + it->nbytes - 1, &last, &unused))
+    return ErrorCode::INVALID_ARGUMENT;
+  it->flags |= flag;
+  it->segs = op.segs + first;
+  it->nsegs = static_cast<uint32_t>(last - first + 1);
+  it->seg_skip = skip;
+  return ErrorCode::OK;
+}
+
 ErrorCode GpuFabric::build_put_items(const std::vector<client::DeviceShardOp>& ops, const std::vector<const void*>& dev_ptrs,
                                      std::vector<XferItem>* items, std::vector<size_t>* op_of_item) {
   items->reserve(ops.size());
   for (size_t k = 0; k < ops.size(); ++k) {
     const auto& op = ops[k];
     XferItem it;
-    it.src = static_cast<const uint8_t*>(dev_ptrs[op.item]) + op.obj_offset;
     it.nbytes = op.placement->length;
+    if (op.segs) {
+      BB_TRY(attach_segments(op, XFER_GATHER, &it));
+    } else {
+      it.src = static_cast<const uint8_t*>(dev_ptrs[op.item]) + op.obj_offset;
+    }
     // NVLS: the replica set is one whole multicast group at one offset -> a single multimem.st stream
     if (arena_ && !op.replicas.empty() && (it.nbytes & 15) == 0) {
       size_t grp = 0, g2 = 0;
@@ -578,6 +598,8 @@ ErrorCode GpuFabric::build_put_items(const std::vector<client::DeviceShardOp>& o
       XferItem more;
       more.src = it.src;
       more.nbytes = it.nbytes;
+      more.flags = it.flags & XFER_GATHER;
+      more.segs = it.segs, more.nsegs = it.nsegs, more.seg_skip = it.seg_skip;
       more.ndst = 0;
       for (; r < op.replicas.size() && more.ndst < kMaxDst; ++r) {
         auto d = resolve(*op.replicas[r]);
@@ -711,11 +733,15 @@ Result<uint64_t> GpuFabric::submit_get(const std::vector<client::DeviceShardOp>&
     auto s = resolve(*op.placement);
     if (!s.ok()) return s.error();
     it.src = s.value();
-    it.dst[0] = static_cast<uint8_t*>(dev_ptrs[op.item]) + op.obj_offset;
     it.ndst = 1;
     it.nbytes = op.placement->length;
     it.expect = op.placement->checksum;
     it.flags = algo == ChecksumAlgo::NONE ? 0u : static_cast<uint32_t>(XFER_VERIFY);
+    if (op.segs) {
+      BB_TRY(attach_segments(op, XFER_SCATTER, &it));
+    } else {
+      it.dst[0] = static_cast<uint8_t*>(dev_ptrs[op.item]) + op.obj_offset;
+    }
     items.push_back(it);
     count(false, classify(*op.placement), it.nbytes);
   }
@@ -763,11 +789,15 @@ ErrorCode GpuFabric::get_shards(const std::vector<client::DeviceShardOp>& ops, c
       auto s = resolve(*op.placement);
       if (!s.ok()) return s.error();
       it.src = s.value();
-      it.dst[0] = static_cast<uint8_t*>(dev_ptrs[op.item]) + op.obj_offset;
       it.ndst = 1;
       it.nbytes = op.placement->length;
       it.expect = op.placement->checksum;
       it.flags = algo == ChecksumAlgo::NONE ? 0u : static_cast<uint32_t>(XFER_VERIFY);
+      if (op.segs) {
+        BB_TRY(attach_segments(op, XFER_SCATTER, &it));
+      } else {
+        it.dst[0] = static_cast<uint8_t*>(dev_ptrs[op.item]) + op.obj_offset;
+      }
       items.push_back(it);
       idx.push_back(k);
     }

@@ -24,8 +24,9 @@ namespace bb::gpu {
   } while (0)
 
 struct XferEngine::Slot {
-  // host (pinned): [descs | tile_start]
+  // host (pinned): [descs | tile_start | segment tables (segmented batches)]
   uint8_t* h_tab = nullptr;
+  size_t tab_cap = 0;  // bytes of h_tab and d_tab (grown on demand by segmented batches)
   // device
   uint8_t* d_tab = nullptr;
   uint64_t* d_sum = nullptr;
@@ -69,6 +70,7 @@ Result<std::unique_ptr<XferEngine>> XferEngine::create(int device, uint32_t max_
     ok = ok && cudaMallocHost(reinterpret_cast<void**>(&s->h_tab), tab_bytes) == cudaSuccess;
     ok = ok && cudaMallocHost(reinterpret_cast<void**>(&s->h_res), res_bytes) == cudaSuccess;
     ok = ok && cudaMalloc(reinterpret_cast<void**>(&s->d_tab), tab_bytes) == cudaSuccess;
+    s->tab_cap = tab_bytes;
     ok = ok && cudaMalloc(reinterpret_cast<void**>(&s->d_sum), static_cast<size_t>(max_items) * 8) == cudaSuccess;
     ok = ok && cudaMalloc(reinterpret_cast<void**>(&s->d_done), static_cast<size_t>(max_items) * 4) == cudaSuccess;
     ok = ok && cudaMalloc(reinterpret_cast<void**>(&s->d_digest), static_cast<size_t>(max_items) * 8) == cudaSuccess;
@@ -253,22 +255,72 @@ Result<uint64_t> XferEngine::submit(const std::vector<XferItem>& items, Checksum
 
   auto run = [&]() -> ErrorCode {
     BB_CUDA(cudaSetDevice(device_));
+    // segmented items: their tables follow the descriptor table and tile_start (sized for every item) in the same
+    // staging buffer, so the batch is still one H2D copy
+    constexpr uint32_t kSegFlags = XFER_GATHER | XFER_SCATTER;
+    const size_t seg_base = (items.size() * sizeof(XferDesc) + (items.size() + 1) * 4 + 15) & ~size_t{15};
+    uint64_t seg_entries = 0;
+    for (const XferItem& it : items)
+      if (it.nbytes && (it.flags & kSegFlags)) seg_entries += static_cast<uint64_t>(it.nsegs) + 1;
+    const bool segmented = seg_entries > 0;
+    if (seg_entries > kMaxSegTableEntries) return ErrorCode::RESOURCE_EXHAUSTED;
+    if (segmented && seg_base + seg_entries * sizeof(XferSeg) > s->tab_cap) {
+      const size_t cap = std::max<size_t>(seg_base + seg_entries * sizeof(XferSeg), 2 * s->tab_cap);
+      cudaFreeHost(s->h_tab);
+      cudaFree(s->d_tab);
+      s->h_tab = nullptr, s->d_tab = nullptr, s->tab_cap = 0;
+      BB_CUDA(cudaMallocHost(reinterpret_cast<void**>(&s->h_tab), cap));
+      BB_CUDA(cudaMalloc(reinterpret_cast<void**>(&s->d_tab), cap));
+      s->tab_cap = cap;
+    }
+    auto* seg_h = reinterpret_cast<XferSeg*>(s->h_tab + seg_base);
+    uint64_t seg_used = 0;
+    // Packs item `it`'s list as one table (header + pieces); returns the table's device address.
+    auto pack_segments = [&](const XferItem& it) -> Result<uint64_t> {
+      if (!it.segs || it.nsegs == 0) return ErrorCode::INVALID_ARGUMENT;
+      XferSeg* t = seg_h + seg_used;
+      uint64_t left = it.nbytes, cnt = 0;
+      for (uint32_t k = 0; k < it.nsegs && left; ++k) {
+        uint64_t p = it.segs[k].ptr, l = it.segs[k].len;
+        if (k == 0) {
+          if (it.seg_skip >= l) return ErrorCode::INVALID_ARGUMENT;
+          p += it.seg_skip, l -= it.seg_skip;
+        }
+        l = std::min(l, left);
+        left -= l;
+        if ((p & 15) || (left && (l & 15))) return ErrorCode::INVALID_ADDRESS;
+        t[++cnt] = XferSeg{p, it.nbytes - left};
+      }
+      if (left) return ErrorCode::INVALID_ARGUMENT;
+      t[0] = XferSeg{cnt, 0};
+      const uint64_t dev = reinterpret_cast<uint64_t>(s->d_tab + seg_base) + seg_used * sizeof(XferSeg);
+      seg_used += cnt + 1;
+      return dev;
+    };
     auto* descs = reinterpret_cast<XferDesc*>(s->h_tab);
     s->item_to_desc.assign(items.size(), -1);
     uint32_t nd = 0, tiles = 0;
-    bool all_small = small_path_enabled();
+    bool all_small = small_path_enabled() && !segmented;
     for (size_t i = 0; i < items.size(); ++i) {
       const XferItem& it = items[i];
       if (it.nbytes == 0) continue;
       all_small = all_small && it.nbytes <= kSmallBytes && !(it.flags & XFER_RAW_SUM) && it.ndst >= 1;
       if (it.ndst > kMaxDst || (it.ndst == 0 && !(it.flags & XFER_RAW_SUM))) return ErrorCode::INVALID_ARGUMENT;
-      uintptr_t al = reinterpret_cast<uintptr_t>(it.src);
-      for (uint32_t r = 0; r < it.ndst; ++r) al |= reinterpret_cast<uintptr_t>(it.dst[r]);
+      const bool gather = it.flags & XFER_GATHER, scatter = it.flags & XFER_SCATTER;
+      if (scatter && (it.ndst != 1 || (it.flags & XFER_MULTIMEM))) return ErrorCode::INVALID_ARGUMENT;
+      uintptr_t al = gather ? 0 : reinterpret_cast<uintptr_t>(it.src);
+      for (uint32_t r = scatter ? 1 : 0; r < it.ndst; ++r) al |= reinterpret_cast<uintptr_t>(it.dst[r]);
       if (al & 15) return ErrorCode::INVALID_ADDRESS;
       if ((it.flags & XFER_MULTIMEM) && (it.nbytes & 15)) return ErrorCode::INVALID_ARGUMENT;
       XferDesc& d = descs[nd];
       d.src = it.src;
       for (uint32_t r = 0; r < kMaxDst; ++r) d.dst[r] = r < it.ndst ? it.dst[r] : nullptr;
+      if (gather || scatter) {
+        auto t = pack_segments(it);
+        if (!t.ok()) return t.error();
+        if (gather) d.src = reinterpret_cast<const void*>(t.value());
+        else d.dst[0] = reinterpret_cast<void*>(t.value());
+      }
       d.nbytes = it.nbytes;
       d.first_tile = tiles;
       d.ndst = it.ndst;
@@ -294,8 +346,9 @@ Result<uint64_t> XferEngine::submit(const std::vector<XferItem>& items, Checksum
     s->debug = capture_debug;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (nd) {
-      const size_t tab = static_cast<size_t>(nd) * sizeof(XferDesc) + (static_cast<size_t>(nd) + 1) * 4;
-      const bool inline_tab = nd <= kInlineDescs;
+      const size_t tab = segmented ? seg_base + seg_used * sizeof(XferSeg)
+                                   : static_cast<size_t>(nd) * sizeof(XferDesc) + (static_cast<size_t>(nd) + 1) * 4;
+      const bool inline_tab = nd <= kInlineDescs && !segmented;
       if (!inline_tab) BB_CUDA(cudaMemcpyAsync(s->d_tab, s->h_tab, tab, cudaMemcpyHostToDevice, st));
       if (capture_debug) {
         const size_t need = static_cast<size_t>(tiles) * tchash::kRows * tchash::kN * 4;
@@ -337,6 +390,7 @@ Result<uint64_t> XferEngine::submit(const std::vector<XferItem>& items, Checksum
       l.max_ctas = max_ctas_;
       l.stream = stream;
       l.small_path = all_small;
+      l.segmented = segmented;
       // Latency path: a small batch whose results land in pinned memory completes by flag -- the launch is the ONLY
       // stream operation (no timing events, no completion event: each costs about as much GPU time as the kernel).
       // (1) resident mailbox warp: no launch at all.  The request bypasses `stream`, so everything already queued there

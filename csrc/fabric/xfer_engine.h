@@ -13,9 +13,16 @@
 #include "common/checksum.h"
 #include "common/error.h"
 #include "common/result.h"
+#include "common/types.h"
 #include "kernels/xfer.h"
 
 namespace bb::gpu {
+
+// One piece of a segmented item (common/types.h).
+using XferSegment = DeviceSegment;
+
+// Segment table entries one launch may carry (segments plus one header per segmented item, kernels/xfer.h XferSeg).
+constexpr uint64_t kMaxSegTableEntries = 1ull << 21;
 
 struct XferItem {
   const void* src = nullptr;
@@ -25,6 +32,13 @@ struct XferItem {
   uint64_t expect = 0;   // expected digest when flags & XFER_VERIFY
   uint32_t flags = 0;
   uint32_t tile_base = 0;  // XFER_RAW_SUM: index of this slice's first tile inside the hashed object
+  // Segmented source (flags & XFER_GATHER, replaces `src`) or destination (flags & XFER_SCATTER, replaces `dst[0]`;
+  // ndst == 1): the item's bytes are segs[0..nsegs) with the first `seg_skip` bytes of segs[0] left out, cut at
+  // `nbytes`.  The list must cover nbytes; every piece must start 16-byte aligned and every piece but the last must be a
+  // multiple of 16 bytes long.  submit() packs the tables after the descriptor table (same H2D copy).
+  const XferSegment* segs = nullptr;
+  uint32_t nsegs = 0;
+  uint64_t seg_skip = 0;
 };
 
 // One object of a fused MXFP8 transfer: `wide` is the caller's bf16 tensor, `packed` the slab location of the

@@ -20,7 +20,24 @@ enum XferFlags : uint32_t {
   // index, so a byte range can be hashed as a slice of a larger object (its sums add up with the slices
   // hashed elsewhere; the host finalises).  With ndst == 0 the descriptor is hash-only (nothing is stored).
   XFER_RAW_SUM = 1u << 2,
+  // Segmented objects: the descriptor's bytes come from (GATHER) or go to (SCATTER) a list of device segments instead of
+  // one contiguous buffer.  GATHER: `src` points to a segment table.  SCATTER: `dst[0]` points to one (ndst == 1, not
+  // with XFER_MULTIMEM).  Digests are those of the concatenated bytes.  Launches that carry either flag must set
+  // XferLaunch::segmented; they never take the warp-per-object kernel, the mailbox or the inline parameter table.
+  XFER_GATHER = 1u << 3,
+  XFER_SCATTER = 1u << 4,
 };
+
+// Segment table of one segmented descriptor (device memory, 16-byte aligned): entry 0 is a header whose `addr` holds
+// the number of segments n and whose `end` is 0; entries 1..n are the segments in order.  `end` is the cumulative byte
+// offset inside the descriptor's range, so segment j covers [table[j-1].end, table[j].end) and table[n].end == nbytes.
+// Every segment starts 16-byte aligned and is non-empty; every segment but the last has a length that is a multiple
+// of 16.  Overlapping scatter destinations get unspecified bytes (never a fault).
+struct XferSeg {
+  uint64_t addr;
+  uint64_t end;
+};
+static_assert(sizeof(XferSeg) == 16);
 
 // 64-byte transfer descriptor, one per (object shard, direction).
 struct XferDesc {
@@ -61,6 +78,7 @@ struct XferLaunch {
   int algo = ALGO_BBH64;
   bool small_path = false;               // every descriptor is <= kSmallBytes, none is a RAW_SUM slice: warp-per-object kernel
   bool flag_completion = false;          // small path only: status_out (pinned, preset to kSmallPending) is the completion flag
+  bool segmented = false;                // some descriptor carries XFER_GATHER / XFER_SCATTER: device tables only
   int max_ctas = 0;                      // 0 = one CTA per SM
   void* stream = nullptr;                // cudaStream_t
 };

@@ -193,7 +193,45 @@ __device__ __forceinline__ uint32_t warp_xpow_tiles(uint32_t k, uint32_t lane) {
   return v;
 }
 
-template <int ALGO>
+// Segment tables (XferSeg, kernels/xfer.h).  Index j >= 1 of the first segment whose end lies past `off`.
+__device__ __forceinline__ uint32_t seg_find(const XferSeg* t, uint64_t off) {
+  uint32_t lo = 1, hi = static_cast<uint32_t>(__ldg(&t[0].addr));
+  while (lo < hi) {
+    const uint32_t mid = (lo + hi) >> 1;
+    if (__ldg(&t[mid].end) > off) hi = mid; else lo = mid + 1;
+  }
+  return lo;
+}
+// Address of object byte `off`, which lies in the table's last segment (the byte tail of an object).
+__device__ __forceinline__ uint64_t seg_last_addr(const XferSeg* t, uint64_t off) {
+  const uint32_t n = static_cast<uint32_t>(__ldg(&t[0].addr));
+  return __ldg(&t[n].addr) + (off - __ldg(&t[n - 1].end));
+}
+// Calls f(global address, tile offset, bytes) once per piece of the 16-byte part [off, off + b16) of a tile, starting at
+// segment `first` (seg_find).  The pieces are spread over the lanes of the warp: lane l takes segments first + l,
+// first + l + 32, ...  Every piece is 16-byte aligned and a multiple of 16 bytes long (the segment rules).
+template <typename F>
+__device__ __forceinline__ void seg_pieces(const XferSeg* t, uint32_t first, uint64_t off, uint32_t b16, uint32_t lane, F&& f) {
+  if (b16 == 0) return;
+  const uint32_t n = static_cast<uint32_t>(__ldg(&t[0].addr));
+  const uint64_t lim = off + b16;
+  for (uint32_t j0 = first;; j0 += 32) {
+    const uint32_t j = j0 + lane;
+    bool more = false;
+    if (j <= n) {
+      const uint64_t sb = __ldg(&t[j - 1].end);
+      if (sb < lim) {
+        const uint64_t se = __ldg(&t[j].end);
+        const uint64_t lo = sb > off ? sb : off, hi = se < lim ? se : lim;
+        f(__ldg(&t[j].addr) + (lo - sb), static_cast<uint32_t>(lo - off), static_cast<uint32_t>(hi - lo));
+        more = true;
+      }
+    }
+    if (!__shfl_sync(0xffffffffu, more ? 1u : 0u, 31)) break;
+  }
+}
+
+template <int ALGO, bool SEG>
 __global__ void __launch_bounds__(kThreads, 1) bb_xfer_kernel(const __grid_constant__ Params p) {
   using Smem = SmemT<ALGO>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -264,7 +302,7 @@ __global__ void __launch_bounds__(kThreads, 1) bb_xfer_kernel(const __grid_const
         uint32_t lo = 0, hi = p.ndesc;  // tile_start[lo] <= t < tile_start[hi]
         uint32_t first, next;
         uint4 q0, q1, q2, q3;
-        if (p.use_inline) {  // table in the parameter space (plain loads: ld.global.nc is illegal there)
+        if (!SEG && p.use_inline) {  // table in the parameter space (plain loads: ld.global.nc is illegal there)
           while (hi - lo > 1) {
             const uint32_t mid = (lo + hi) >> 1;
             if (p.inl_tile_start[mid] <= t) lo = mid; else hi = mid;
@@ -295,6 +333,13 @@ __global__ void __launch_bounds__(kThreads, 1) bb_xfer_kernel(const __grid_const
         e.m.ndst_flags = (q2.w & 0xFFu) | (q3.z << 8);
         e.m.obj_ntiles = next - first;
         e.m.crc_unpad = q3.w;
+        if constexpr (SEG) {
+          // first segment of this tile, looked up for 32 tiles at once: the gather index rides in the entry's spare word,
+          // the scatter index in dst[1] (a scatter descriptor has one destination)
+          const uint64_t toff = static_cast<uint64_t>(t - first) * kTileBytes;
+          if (q3.z & XFER_GATHER) e.pad = seg_find(reinterpret_cast<const XferSeg*>(e.src), toff);
+          if (q3.z & XFER_SCATTER) e.m.dst[1] = seg_find(reinterpret_cast<const XferSeg*>(e.m.dst[0]), toff);
+        }
       }
       __syncwarp();
       const uint32_t cnt = min(32u, my_tiles - base);
@@ -307,6 +352,7 @@ __global__ void __launch_bounds__(kThreads, 1) bb_xfer_kernel(const __grid_const
         const uint32_t bytes = static_cast<uint32_t>(min(static_cast<uint64_t>(kTileBytes), e.m.nbytes - off));
         const uint32_t b16 = bytes & ~15u;
         const uint32_t tail = bytes & 15u;
+        const bool gather = SEG && ((e.m.ndst_flags >> 8) & XFER_GATHER);
         mbar_wait(&s.empty[stage], par ^ 1u);
         bool wrote = false;
         if constexpr (kHash) {
@@ -317,7 +363,12 @@ __global__ void __launch_bounds__(kThreads, 1) bb_xfer_kernel(const __grid_const
           }
         }
         if (lane < tail) {
-          s.tile[stage][b16 + lane] = *reinterpret_cast<const uint8_t*>(src_i + off + b16 + lane);
+          if constexpr (SEG) {
+            const uint64_t a = gather ? seg_last_addr(reinterpret_cast<const XferSeg*>(src_i), off + b16) : src_i + off + b16;
+            s.tile[stage][b16 + lane] = *reinterpret_cast<const uint8_t*>(a + lane);
+          } else {
+            s.tile[stage][b16 + lane] = *reinterpret_cast<const uint8_t*>(src_i + off + b16 + lane);
+          }
           wrote = true;
         }
         if (wrote) fence_proxy_async_smem();
@@ -330,8 +381,17 @@ __global__ void __launch_bounds__(kThreads, 1) bb_xfer_kernel(const __grid_const
         if (lane == 0) {
           s.dirty[stage] = (bytes + 15u) & ~15u;
           mbar_arrive_expect_tx(&s.full[stage], b16);
-          if (b16) bulk_g2s(s.tile[stage], reinterpret_cast<const void*>(src_i + off), b16, &s.full[stage]);
+          if (b16 && !gather) bulk_g2s(s.tile[stage], reinterpret_cast<const void*>(src_i + off), b16, &s.full[stage]);
           if (p.trace_d) p.trace_d[static_cast<uint64_t>(t0 + base + i) * 4 + 0] = globaltimer_ns();
+        }
+        if constexpr (SEG) {
+          if (gather) {  // one bulk copy per piece, all completing on the stage's barrier (armed above with the b16 total)
+            __syncwarp();
+            const uint32_t first = static_cast<uint32_t>(e.pad);
+            seg_pieces(reinterpret_cast<const XferSeg*>(src_i), first, off, b16, lane, [&](uint64_t g, uint32_t to, uint32_t nb) {
+              bulk_g2s(&s.tile[stage][to], reinterpret_cast<const void*>(g), nb, &s.full[stage]);
+            });
+          }
         }
         __syncwarp();
       }
@@ -374,26 +434,51 @@ __global__ void __launch_bounds__(kThreads, 1) bb_xfer_kernel(const __grid_const
       const uint32_t tail = m.bytes & 15u;
       const uint32_t ndst = m.ndst_flags & 0xFFu;
       const uint32_t flags = m.ndst_flags >> 8;
+      // scatter: dst[0] is the segment table, dst[1] the first segment of this tile; any lane may issue a piece, so in
+      // the segmented kernel every lane keeps its own bulk groups (commit / wait below)
+      const bool scatter = SEG && (flags & XFER_SCATTER);
       if (flags & XFER_MULTIMEM) {
         uint8_t* mc = reinterpret_cast<uint8_t*>(m.dst[0] + off);
         for (uint32_t o = lane * 16; o < b16; o += 512)
           multimem_st_v4(mc + o, *reinterpret_cast<const uint4*>(&s.tile[stage][o]));
+      } else if (scatter) {
+        seg_pieces(reinterpret_cast<const XferSeg*>(m.dst[0]), static_cast<uint32_t>(m.dst[1]), off, b16, lane,
+                   [&](uint64_t g, uint32_t to, uint32_t nb) { bulk_s2g(reinterpret_cast<void*>(g), &s.tile[stage][to], nb); });
       } else if (lane == 0) {
         for (uint32_t r = 0; r < ndst; ++r)
           if (b16) bulk_s2g(reinterpret_cast<void*>(m.dst[r] + off), s.tile[stage], b16);
       }
-      if (lane == 0) bulk_commit();
+      if (SEG || lane == 0) bulk_commit();
       if (p.trace_d && lane == 0) p.trace_d[static_cast<uint64_t>(t0 + it) * 4 + 2] = globaltimer_ns();
       if (lane < tail) {
         const uint8_t b = s.tile[stage][b16 + lane];
-        for (uint32_t r = 0; r < ndst; ++r) *reinterpret_cast<uint8_t*>(m.dst[r] + off + b16 + lane) = b;
+        if (scatter) {
+          *reinterpret_cast<uint8_t*>(seg_last_addr(reinterpret_cast<const XferSeg*>(m.dst[0]), off + b16) + lane) = b;
+        } else {
+          for (uint32_t r = 0; r < ndst; ++r) *reinterpret_cast<uint8_t*>(m.dst[r] + off + b16 + lane) = b;
+        }
       }
       __syncwarp();
-      if (it >= kStoreLag && lane == 0) {
-        bulk_wait_read<kStoreLag>();
-        mbar_arrive(&s.empty[(it - kStoreLag) % kStages]);
-        if (p.trace_d) p.trace_d[static_cast<uint64_t>(t0 + it - kStoreLag) * 4 + 3] = globaltimer_ns();
+      if constexpr (SEG) {
+        if (it >= kStoreLag) {
+          bulk_wait_read<kStoreLag>();
+          __syncwarp();
+          if (lane == 0) {
+            mbar_arrive(&s.empty[(it - kStoreLag) % kStages]);
+            if (p.trace_d) p.trace_d[static_cast<uint64_t>(t0 + it - kStoreLag) * 4 + 3] = globaltimer_ns();
+          }
+        }
+      } else {
+        if (it >= kStoreLag && lane == 0) {
+          bulk_wait_read<kStoreLag>();
+          mbar_arrive(&s.empty[(it - kStoreLag) % kStages]);
+          if (p.trace_d) p.trace_d[static_cast<uint64_t>(t0 + it - kStoreLag) * 4 + 3] = globaltimer_ns();
+        }
       }
+    }
+    if constexpr (SEG) {
+      bulk_wait_read<0>();
+      __syncwarp();
     }
     if (lane == 0) {
       bulk_wait_read<0>();
@@ -404,6 +489,7 @@ __global__ void __launch_bounds__(kThreads, 1) bb_xfer_kernel(const __grid_const
       }
       bulk_wait<0>();  // writes performed before the kernel retires
     }
+    if constexpr (SEG) bulk_wait<0>();
   } else if (warp == 3) {
     // ================================================================ finalizer
     if constexpr (kHash) {
@@ -646,21 +732,32 @@ struct DeviceState {
   bool consts = false;
   uint32_t* crc_tables = nullptr;
   int sm_count = 0;
-  bool attr[4] = {false, false, false, false};
+  bool attr[4][2] = {};
 };
 DeviceState g_dev[16];
 std::mutex g_mu;
 
-template <int ALGO>
+template <int ALGO, bool SEG>
 cudaError_t launch_t(DeviceState& ds, const Params& p, int grid, cudaStream_t st) {
-  if (!ds.attr[ALGO]) {
-    cudaError_t e = cudaFuncSetAttribute(bb_xfer_kernel<ALGO>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  if (!ds.attr[ALGO][SEG]) {
+    cudaError_t e = cudaFuncSetAttribute(bb_xfer_kernel<ALGO, SEG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          static_cast<int>(sizeof(SmemT<ALGO>)));
     if (e != cudaSuccess) return e;
-    ds.attr[ALGO] = true;
+    ds.attr[ALGO][SEG] = true;
   }
-  bb_xfer_kernel<ALGO><<<grid, kThreads, sizeof(SmemT<ALGO>), st>>>(p);
+  bb_xfer_kernel<ALGO, SEG><<<grid, kThreads, sizeof(SmemT<ALGO>), st>>>(p);
   return cudaGetLastError();
+}
+
+template <bool SEG>
+cudaError_t launch_algo(DeviceState& ds, int algo, const Params& p, int grid, cudaStream_t st) {
+  switch (algo) {
+    case ALGO_NONE: return launch_t<ALGO_NONE, SEG>(ds, p, grid, st);
+    case ALGO_CRC32C: return launch_t<ALGO_CRC32C, SEG>(ds, p, grid, st);
+    case ALGO_BBH64: return launch_t<ALGO_BBH64, SEG>(ds, p, grid, st);
+    case ALGO_XXH3: return launch_t<ALGO_XXH3, SEG>(ds, p, grid, st);
+    default: return cudaErrorNotSupported;
+  }
 }
 
 }  // namespace
@@ -718,7 +815,8 @@ uint32_t crc_init_term_for(uint64_t nbytes) {
 
 int launch_xfer(const XferLaunch& l) {
   if (l.ndesc == 0 || l.total_tiles == 0) return 0;
-  if (l.small_path && !l.debug_d && !l.trace_d) return launch_xfer_small(l);
+  if (l.small_path && !l.segmented && !l.debug_d && !l.trace_d) return launch_xfer_small(l);
+  if (l.segmented && (!l.descs || !l.tile_start)) return static_cast<int>(cudaErrorInvalidValue);
   int dev = 0;
   cudaError_t e = cudaGetDevice(&dev);
   if (e != cudaSuccess) return static_cast<int>(e);
@@ -763,7 +861,7 @@ int launch_xfer(const XferLaunch& l) {
   p.descs = l.descs;
   p.tile_start = l.tile_start;
   p.use_inline = 0;
-  if (l.host_descs && l.ndesc <= kInlineDescs) {
+  if (l.host_descs && l.ndesc <= kInlineDescs && !l.segmented) {
     p.use_inline = 1;
     std::memcpy(p.inl_descs, l.host_descs, l.ndesc * sizeof(XferDesc));
     std::memcpy(p.inl_tile_start, l.host_tile_start, (l.ndesc + 1) * sizeof(uint32_t));
@@ -784,13 +882,7 @@ int launch_xfer(const XferLaunch& l) {
   int grid = l.max_ctas > 0 ? l.max_ctas : env_ctas > 0 ? env_ctas : l.algo == ALGO_CRC32C ? ds.sm_count : std::min(ds.sm_count, 128);
   grid = static_cast<int>(std::min<uint32_t>(static_cast<uint32_t>(grid), l.total_tiles));
   cudaStream_t st = static_cast<cudaStream_t>(l.stream);
-  switch (l.algo) {
-    case ALGO_NONE: e = launch_t<ALGO_NONE>(ds, p, grid, st); break;
-    case ALGO_CRC32C: e = launch_t<ALGO_CRC32C>(ds, p, grid, st); break;
-    case ALGO_BBH64: e = launch_t<ALGO_BBH64>(ds, p, grid, st); break;
-    case ALGO_XXH3: e = launch_t<ALGO_XXH3>(ds, p, grid, st); break;
-    default: return static_cast<int>(cudaErrorNotSupported);
-  }
+  e = l.segmented ? launch_algo<true>(ds, l.algo, p, grid, st) : launch_algo<false>(ds, l.algo, p, grid, st);
   return static_cast<int>(e);
 }
 

@@ -12,6 +12,7 @@
 #include "coord/etcd_coord.h"
 #include "coord/coord.h"
 #include "keystone/keystone_service.h"
+#include "py/segments.h"
 #include "rpc/rpc_service.h"
 #include "rpc/wire.h"
 #include "worker/worker_service.h"
@@ -1196,6 +1197,24 @@ void bind_control(py::module_& m) {
         }
         return py::make_tuple(ecs_to_py(ecs), sizes);
       }, py::arg("keys"), py::arg("dev_ptrs"), py::arg("capacity"), py::arg("stream") = 0)
+      .def("batch_put_device_gather", [](BlackbirdClient& c, const std::vector<std::string>& keys, const py::handle& segs,
+                                         const std::vector<uint32_t>& seg_counts, const WorkerConfig& cfg, uintptr_t stream) {
+        auto a = py_segments::read_segments(segs);
+        std::vector<DeviceSegment> v(a.count);
+        if (a.count) std::memcpy(v.data(), a.data, a.count * sizeof(DeviceSegment));
+        return ecs_to_py(nogil([&] { return c.batch_put_device_gather(keys, v, seg_counts, cfg, reinterpret_cast<void*>(stream)); }));
+      }, py::arg("keys"), py::arg("segs"), py::arg("seg_counts"), py::arg("config") = WorkerConfig{}, py::arg("stream") = 0,
+         "Segmented put: object i is the concatenation of the next seg_counts[i] rows (device pointer, bytes) of the (S, 2) "
+         "uint64 / int64 array `segs`.  Stored exactly as a contiguous put of that concatenation.")
+      .def("batch_get_device_scatter", [](BlackbirdClient& c, const std::vector<std::string>& keys, const py::handle& segs,
+                                          const std::vector<uint32_t>& seg_counts, uintptr_t stream) {
+        auto a = py_segments::read_segments(segs);
+        std::vector<DeviceSegment> v(a.count);
+        if (a.count) std::memcpy(v.data(), a.data, a.count * sizeof(DeviceSegment));
+        return ecs_to_py(nogil([&] { return c.batch_get_device_scatter(keys, v, seg_counts, reinterpret_cast<void*>(stream)); }));
+      }, py::arg("keys"), py::arg("segs"), py::arg("seg_counts"), py::arg("stream") = 0,
+         "Segmented get: object i is scattered over the next seg_counts[i] rows of `segs`; their lengths must add up to the "
+         "stored size.")
       .def("cluster_stats", [](BlackbirdClient& c) { return unwrap(nogil([&] { return c.cluster_stats(); })); })
       .def("metrics_text", &BlackbirdClient::metrics_text)
       .def("set_device_pipeline_chunks", &BlackbirdClient::set_device_pipeline_chunks)

@@ -8,6 +8,9 @@
 #include "fabric/gpu_fabric.h"
 #include "fabric/xfer_engine.h"
 #include "kernels/xfer.h"
+#include "py/segments.h"
+
+#include <deque>
 
 namespace py = pybind11;
 using namespace bb;
@@ -20,13 +23,29 @@ void check(ErrorCode ec, const char* what) {
 void check_cuda(int rc, const char* what) {
   if (rc != 0) throw std::runtime_error(std::string(what) + ": CUDA error " + std::to_string(rc) + " " + cuda_error_string(rc));
 }
-// item tuple: (src, dst | [dst...], nbytes, expect=0, flags=0)
-XferItem to_item(const py::handle& h) {
+// item tuple: (src | segments, dst | [dst...] | segments, nbytes, expect=0, flags=0).  `segments` = an (S, 2) array of
+// (device pointer, bytes) rows (py/segments.h): a gathered source or a scattered destination.  `keep` holds the arrays
+// until the batch is submitted (the engine copies the tables into its staging buffer).
+XferItem to_item(const py::handle& h, std::deque<py_segments::SegmentArray>& keep) {
   py::tuple t = py::cast<py::tuple>(h);
-  if (t.size() < 3) throw py::value_error("xfer item = (src, dst|[dst..], nbytes[, expect[, flags]])");
+  if (t.size() < 3) throw py::value_error("xfer item = (src|segments, dst|[dst..]|segments, nbytes[, expect[, flags]])");
   XferItem it;
-  it.src = reinterpret_cast<const void*>(t[0].cast<uintptr_t>());
-  if (py::isinstance<py::int_>(t[1])) {
+  if (py_segments::is_segment_array(t[0])) {
+    keep.push_back(py_segments::read_segments(t[0]));
+    it.segs = keep.back().data;
+    it.nsegs = static_cast<uint32_t>(keep.back().count);
+    it.flags |= XFER_GATHER;
+  } else {
+    it.src = reinterpret_cast<const void*>(t[0].cast<uintptr_t>());
+  }
+  if (py_segments::is_segment_array(t[1])) {
+    if (it.segs) throw py::value_error("an item gathers or scatters, not both");
+    keep.push_back(py_segments::read_segments(t[1]));
+    it.segs = keep.back().data;
+    it.nsegs = static_cast<uint32_t>(keep.back().count);
+    it.flags |= XFER_SCATTER;
+    it.ndst = 1;
+  } else if (py::isinstance<py::int_>(t[1])) {
     it.dst[0] = reinterpret_cast<void*>(t[1].cast<uintptr_t>());
     it.ndst = 1;
   } else {
@@ -37,7 +56,7 @@ XferItem to_item(const py::handle& h) {
   }
   it.nbytes = t[2].cast<uint64_t>();
   if (t.size() > 3) it.expect = t[3].cast<uint64_t>();
-  if (t.size() > 4) it.flags = t[4].cast<uint32_t>();
+  if (t.size() > 4) it.flags |= t[4].cast<uint32_t>();
   return it;
 }
 }  // namespace
@@ -46,6 +65,8 @@ void bind_gpu(py::module_& m) {
   m.attr("TILE_BYTES") = kTileBytes;
   m.attr("XFER_VERIFY") = static_cast<uint32_t>(XFER_VERIFY);
   m.attr("XFER_MULTIMEM") = static_cast<uint32_t>(XFER_MULTIMEM);
+  m.attr("XFER_GATHER") = static_cast<uint32_t>(XFER_GATHER);
+  m.attr("XFER_SCATTER") = static_cast<uint32_t>(XFER_SCATTER);
   m.def("cuda_device_count", [] {
     int n = 0;
     device_count(&n);
@@ -62,8 +83,9 @@ void bind_gpu(py::module_& m) {
       .def("run",
            [](XferEngine& e, const py::list& items, ChecksumAlgo algo, uintptr_t stream, bool debug) {
              std::vector<XferItem> v;
+             std::deque<py_segments::SegmentArray> keep;
              v.reserve(items.size());
-             for (auto h : items) v.push_back(to_item(h));
+             for (auto h : items) v.push_back(to_item(h, keep));
              XferResult res;
              {
                py::gil_scoped_release rel;
@@ -112,8 +134,9 @@ void bind_gpu(py::module_& m) {
       .def("submit",
            [](XferEngine& e, const py::list& items, ChecksumAlgo algo, uintptr_t stream) {
              std::vector<XferItem> v;
+             std::deque<py_segments::SegmentArray> keep;
              v.reserve(items.size());
-             for (auto h : items) v.push_back(to_item(h));
+             for (auto h : items) v.push_back(to_item(h, keep));
              auto t = e.submit(v, algo, reinterpret_cast<void*>(stream));
              if (!t.ok()) check(t.error(), "XferEngine.submit");
              return t.value();
